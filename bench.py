@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Benchmark of the LAVT-RS hot path on B200:  python bench.py --gpus N --steps K --warmup W
+"""Benchmark of the LAVT-RS hot path on B200:  python bench.py --gpus N --steps K --warmup W [--dump-outputs DIR]
 
 Metric (BASELINE.json): LAVT-RS forward clips/s on 8x384x384 clips, Video Swin-B, 20-word expression.
 One step = one ``LAVTVideo.forward(x, text ids, l_mask)`` (BERT-base text encoder + backbone + PWAM/gate + SimpleDecoding +
@@ -35,8 +35,13 @@ T_FRAMES, IMG, NL = 8, 384, 20
 def parse():
     p = argparse.ArgumentParser()
     p.add_argument("--gpus", type=int, default=1)
-    p.add_argument("--steps", type=int, default=10)
+    p.add_argument("--steps", type=_positive, default=10)
     p.add_argument("--warmup", type=int, default=3)
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the logits of the last timed step to DIR/logits.npy as float32; an output "
+                        "over 64 MB is cut to a seeded choice of whole frames, listed in the JSON line under dump_outputs.  With "
+                        "WORLD_SIZE > 1 only rank 0's clips are written.  --impl reference times one clip of other inputs, so its "
+                        "dump compares only with another --impl reference dump")
     p.add_argument("--impl", default="b200", choices=["b200", "reference"])
     p.add_argument("--clips-per-gpu", type=int, default=8)
     p.add_argument("--window12", action="store_true", help="(8,12,12) windows instead of the default (8,7,7)")
@@ -49,6 +54,30 @@ def parse():
                    help="skip the extra keys of the N=1 line: gpu_eager_baseline (the oracle port run as eager PyTorch on this GPU, fp32 and "
                         "bf16 autocast), latency_1clip (BASELINE configs[1] is literally one clip), window12 / sep_t_pwam throughput")
     return p.parse_args()
+
+
+def _positive(s: str) -> int:
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1")
+    return v
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_logits(out: torch.Tensor, d: str) -> dict:
+    """Write ``out`` (n_frames, 2, H, W) as float32 to ``d``/logits.npy.  Over DUMP_BYTES, a seeded, sorted choice of whole frames is
+    kept, so that two builds given the same arguments write the same frames."""
+    import numpy as np
+    n = out.shape[0]
+    per_frame = out[0].numel() * 4
+    keep = min(n, DUMP_BYTES // per_frame)
+    frames = torch.arange(n) if keep == n else torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    arr = out[frames.to(out.device)].float().cpu().numpy()
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "logits.npy"), arr)
+    return {"logits": {"shape": list(arr.shape), "of_shape": list(out.shape), "frames": frames.tolist()}}
 
 
 SEP_T_PWAM = False      # set from --sep-t-pwam in main()
@@ -332,14 +361,14 @@ def run_reference(a):
     torch.manual_seed(0)
     model = segmentation.lavt_video(pretrained="", args=model_args(a.window12)).eval()
     sd = {k: v.detach().float() for k, v in model.state_dict().items()}
-    budget_s = 200.0
     warm = min(a.warmup, 1)
-    wt, _, _ = cpu_forward_time(a.window12, sd, max(warm, 1), threads)
-    steps = max(1, min(a.steps, int(budget_s / max(wt[-1], 1e-3))))
-    times, _, _ = cpu_forward_time(a.window12, sd, steps, threads)
+    cpu_forward_time(a.window12, sd, max(warm, 1), threads)
+    steps = a.steps
+    times, out, _ = cpu_forward_time(a.window12, sd, steps, threads)
     per = sum(times) / len(times)
     v = 1.0 / per
-    sample = f"1 clip (8x384x384) per step, {steps} of {a.steps} requested steps timed after {max(warm,1)} warm-up, fp32, torch CPU"
+    sample = f"1 clip (8x384x384) per step, {steps} steps timed after {max(warm,1)} warm-up, fp32, torch CPU"
+    dumped = dump_logits(out, a.dump_outputs) if a.dump_outputs else None
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": "clips/s", "n_gpus": a.gpus, "steps": steps,
         "warmup": max(warm, 1), "ms_per_step": per * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -348,6 +377,7 @@ def run_reference(a):
                    "window": "8x12x12" if a.window12 else "8x7x7", "clips_per_step": 1},
         "cpu_baseline": {"value": v, "unit": "clips/s", "cores": threads, "kind": "port", "sample": sample},
         "e2e": {"value": v, "unit": "clips/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
+        **({"dump_outputs": dumped} if dumped else {}),
     }))
 
 
@@ -406,12 +436,13 @@ def main():
                 out = fwd_static()
 
         def step_resident(i):
+            nonlocal out
             rx, rl, rm = resident[i % 2]
             sx.copy_(rx); sl.copy_(rl); sm_.copy_(rm)       # device-to-device refresh of the static inputs (part of the step)
             if graph is not None:
-                graph.replay()
+                graph.replay()                              # writes the captured ``out``
             else:
-                fwd_static()
+                out = fwd_static()
 
         host_out = torch.empty(out.shape, dtype=out.dtype).pin_memory()
 
@@ -493,6 +524,7 @@ def main():
             clocks.start()
         ms = timed(step_resident, a.steps, max(a.warmup, 3))
         clk = clocks.stop() if rank == 0 else None
+        dumped = dump_logits(out, a.dump_outputs) if a.dump_outputs and rank == 0 else None
         ms_e2e = timed(step_e2e, a.steps, 1, finish_e2e)
 
         # --- roofline leg: per-launch CUDA events around the dominant kernel families (eager, same inputs) ---
@@ -570,6 +602,8 @@ def main():
         "roofline": roofline,
         "workspace_bytes": E.workspace(dev).bytes(),
     }
+    if dumped:
+        res["dump_outputs"] = dumped
 
     if world == 1 and not a.no_cpu_baseline:
         threads = os.cpu_count() or 1

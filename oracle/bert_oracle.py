@@ -3,7 +3,7 @@
 
 TEST INFRASTRUCTURE ONLY -- imported by tests/, __graft_entry__.smoke() and bench.py's CPU legs, never by the product path.
 
-The reference's ``bert/`` package is absent from /root/reference: it is a copy of HuggingFace Transformers **v3.0.2**
+The reference's ``bert/`` package is absent from the reference checkout: it is a copy of HuggingFace Transformers **v3.0.2**
 ``modeling_bert.py`` (README.md:9-13), i.e. a third-party dependency.  This file restates that published algorithm
 (BertEmbeddings -> 12 x [BertSelfAttention, BertSelfOutput, BertIntermediate, BertOutput]), and is pinned in
 tests/test_bert_oracle.py against the ``transformers`` BertModel installed here (same architecture and state-dict keys)

@@ -6,9 +6,9 @@ and ``bench.py``'s CPU-baseline / ``--impl reference`` legs may import this modu
 path (``lavt_rs_b200``) never does and has no CPU fallback.
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md section 4), so the oracle
-is pinned against the reference ITSELF, imported unmodified from /root/reference with the shims in
+is pinned against the reference ITSELF, imported unmodified from its checkout with the shims in
 ``oracle/ref_shims.py``: ``oracle/make_golden.py`` runs both on seeded inputs, asserts agreement
-(tests/test_oracle_vs_reference.py does the same whenever /root/reference is present) and stores
+(tests/test_oracle_vs_reference.py does the same whenever that checkout is present) and stores
 small reference outputs under ``tests/golden/`` for the GPU box, where the reference is absent.
 
 Everything is channels-last and index-math based (no roll / partition copies) so that it doubles as

@@ -1,6 +1,6 @@
 """Golden outputs of the UNMODIFIED reference VLT head (lib/vlt.py: VLTFuseAndClassify) -> tests/golden/vlt_*.npz.
 
-    python oracle/make_golden_vlt.py            (build container only: imports /root/reference through oracle/ref_shims.py)
+    python oracle/make_golden_vlt.py            (imports the reference checkout through oracle/ref_shims.py)
 
 Weights: a seeded state dict built with this repo's parameter container (same names / shapes as the reference's module, checked by
 load_state_dict(strict=True) into the reference head), norms and BatchNorm statistics randomised so that every affine / running

@@ -3,8 +3,9 @@
 The reference does not import as shipped (SURVEY.md section 8c): ``timm``, ``mmcv``, ``mmseg`` and its
 ``bert/`` directory are absent and ``MultiModalSwinTransformer3D.__init__`` reads an undefined global
 ``sr_ratio``.  Everything is fixed from OUTSIDE with stub modules; no reference file is edited or copied.
-Used only where /root/reference exists (this container): to pin ``oracle/lavt_oracle.py`` and to
-generate ``tests/golden/*`` (oracle/make_golden.py).  The GPU box never sees the reference.
+Used only where a checkout of the reference is present, in ``oracle/_ref`` (not tracked) or at
+``$LAVT_REFERENCE_ROOT``: to pin ``oracle/lavt_oracle.py`` and to generate ``tests/golden/*``
+(oracle/make_golden.py).  Without it the tests that import the reference skip.
 """
 from __future__ import annotations
 
@@ -15,7 +16,7 @@ import types
 import torch
 import torch.nn as nn
 
-REFERENCE_ROOT = os.environ.get("LAVT_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("LAVT_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 
 def reference_available() -> bool:

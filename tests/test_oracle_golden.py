@@ -1,5 +1,5 @@
 """Oracle (CPU) vs golden outputs produced by the UNMODIFIED reference (oracle/make_golden.py).  This is the pin that
-travels: it runs wherever the repo is, with no access to /root/reference."""
+travels: it runs wherever the repo is, with no checkout of the reference."""
 import os
 import sys
 
@@ -10,7 +10,7 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from oracle import lavt_oracle as O  # noqa: E402
-from oracle.make_golden import CASES, OUT, case_inputs, subsample  # noqa: E402
+from oracle.make_golden import CASES, OUT, case_inputs, subsample, subsample_mask  # noqa: E402
 
 
 @pytest.mark.parametrize("name", sorted(CASES))
@@ -28,8 +28,9 @@ def test_oracle_reproduces_reference_outputs(name):
             key = f"c{i + 1}"
             assert np.abs(subsample(key, cap[key]).numpy() - gold[key]).max() < 5e-4 * max(1.0, np.abs(gold[key]).max()), key
             assert abs(cap[key].norm().item() - float(gold[key + "_norm"])) < 1e-4 * float(gold[key + "_norm"]), key
-        mask = np.unpackbits(gold["mask_bits"])[: logits[:, 0].numel()].reshape(logits[:, 0].shape).astype(bool)
-        agree = ((logits[:, 1] > logits[:, 0]).numpy() == mask).mean()
+        ours = subsample_mask(logits[:, 1] > logits[:, 0]).numpy()
+        mask = np.unpackbits(gold["mask_bits"])[: ours.size].reshape(ours.shape).astype(bool)
+        agree = (ours == mask).mean()
         assert agree >= 0.9999, agree          # fp32 vs fp32: only exact ties can differ
         return
     # EFN ends in an InstanceNorm over nearly uniform co-attention averages at random init: fp32 summation order shows at 2e-3 (see
@@ -48,15 +49,24 @@ def test_oracle_reproduces_reference_outputs(name):
 
 def test_oracle_autograd_reproduces_reference_training_step():
     """Golden training step of the UNMODIFIED reference (oracle/make_golden_train.py): loss, d l_feats, the norm of every parameter
-    gradient and ten complete gradient tensors vs autograd through the oracle."""
+    gradient and ten gradient tensors (leading output channels of the largest) vs autograd through the oracle."""
     from oracle.make_golden_train import TRAIN_CASES, train_case_inputs
     for name, c in TRAIN_CASES.items():
         gold = np.load(os.path.join(OUT, name + ".npz"))
         cfg, sd, x, l, m, target = train_case_inputs(c)
         leaf = {k: v.clone().requires_grad_(v.is_floating_point() and "running" not in k) for k, v in sd.items()}
         lr = l.clone().requires_grad_()
-        loss = O.weighted_cross_entropy(O.model_forward(leaf, cfg, x, lr, m, train_bn=True), target)
-        loss.backward()
+        # A few decoder ReLU inputs of this case lie within fp32 rounding of zero.  The branch they take moves the stage gradients by
+        # ~1e-2 and follows the summation order of the CPU kernels, which changes with the thread count (16 threads fail the bounds
+        # below, 1 / 3 / 8 pass on AVX-512 Xeons).  One thread makes the order independent of the core count; it still depends on the
+        # CPU's instruction set and the kernels torch picks for it.  A case free of such near-ties needs the reference to regenerate.
+        threads = torch.get_num_threads()
+        torch.set_num_threads(1)
+        try:
+            loss = O.weighted_cross_entropy(O.model_forward(leaf, cfg, x, lr, m, train_bn=True), target)
+            loss.backward()
+        finally:
+            torch.set_num_threads(threads)
         assert abs(loss.item() - float(gold["loss"])) < 1e-5
         assert np.abs(lr.grad.numpy() - gold["dl"]).max() < 1e-6 + 2e-3 * np.abs(gold["dl"]).max()
         for k, nrm in zip(gold["names"], gold["norms"]):
@@ -64,7 +74,8 @@ def test_oracle_autograd_reproduces_reference_training_step():
             assert g is not None and abs(g.norm().item() - float(nrm)) < 5e-3 * float(nrm) + 1e-8, k
         for key in gold.files:
             if key.startswith("g:"):
-                a, b = leaf[key[2:]].grad.numpy(), gold[key]
+                b = gold[key]
+                a = leaf[key[2:]].grad.numpy()[: b.shape[0]]
                 assert np.linalg.norm(a - b) < 5e-3 * np.linalg.norm(b) + 1e-9, key
 
 

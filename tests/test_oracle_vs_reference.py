@@ -1,6 +1,7 @@
-"""Pin the oracle (oracle/lavt_oracle.py) against the UNMODIFIED reference modules, imported from
-/root/reference with external shims.  Runs only where the reference tree exists (the build container);
-on the GPU box the same pinning is carried by tests/golden (see test_oracle_golden.py)."""
+"""Pin the oracle (oracle/lavt_oracle.py) against the UNMODIFIED reference modules, imported from a
+checkout of the reference (oracle/_ref or $LAVT_REFERENCE_ROOT, see oracle/ref_shims.py) with external
+shims.  Runs only where that checkout exists; elsewhere the pinning of the forward and training step
+is carried by tests/golden (see test_oracle_golden.py)."""
 import os
 import sys
 
