@@ -129,16 +129,17 @@ int lavt_patch_embed_im2col(const float* x, int64_t stride_b, int64_t stride_c, 
 int lavt_window_attention(const void* qkv, const float* table_t, int32_t L, int32_t nH, const lavt_win_geom_t* geom,
                           void* out_bf16, void* stream);
 /* Same, and lse fp32 [B*nW*N, nH] = log2-sum-exp2 of every score row (what the backward needs besides qkv and out; written by the
- * tcgen05 kernel only -- lavt_window_attention_has_lse tells whether this geometry gets it: 1 / 0). */
+ * tcgen05 kernels only, i.e. for windows of 16 tokens or more -- lavt_window_attention_has_lse tells whether this geometry gets it: 1 / 0). */
 int lavt_window_attention_lse(const void* qkv, const float* table_t, int32_t L, int32_t nH, const lavt_win_geom_t* geom, void* out_bf16,
                               float* lse, void* stream);
 int lavt_window_attention_has_lse(const lavt_win_geom_t* geom, int32_t L, int32_t nH);
-/* Kernel selection for lavt_window_attention (process-wide; initial value from the LAVT_ATTN_IMPL environment variable):
- *   0 = auto: one-pass key-chunked tcgen05 / TMEM kernel (attn_tc2.cu) for windows of up to 1152 tokens
- *   1 = mma.sync kernels only
- *   2 = prefer the two-pass tcgen05 kernel (attn_tc.cu) for windows of <= 400 tokens
- *   3 = attn_tc2.cu (key-chunked one-pass kernel, any window up to 1152 tokens)
- *   4 = attn_tc3.cu (7 x 7 windows: row-parallel warpgroups, run-padded keys; what auto picks for them).  Returns the previous setting. */
+/* Kernel selection for lavt_window_attention (process-wide; initial value from the LAVT_ATTN_IMPL environment variable, "tc2" / "tc3"):
+ *   0 = auto: attn_tc3.cu (row-parallel tcgen05 / TMEM kernel) for windows whose (h, w) extent is the full 7 x 7 or 12 x 12, the
+ *       key-chunked one-pass tcgen05 kernel (attn_tc2.cu) for every other window of 16 ... 1152 tokens, the mma.sync kernel
+ *       (attn_window.cu) for windows of fewer than 16 tokens
+ *   3 = attn_tc2.cu wherever it applies (A/B runs), else as auto
+ *   4 = same as auto (attn_tc3.cu where it applies)
+ * Any other value, including the retired 1 (mma.sync only) and 2 (round-1 tcgen05 kernel), means auto.  Returns the previous setting. */
 int lavt_set_attention_impl(int32_t impl);
 
 /* ---- PWAM (lib/video_swin_transformer.py:919-1009) ---- */

@@ -427,11 +427,14 @@ def patch_embed_im2col(x: torch.Tensor, out_bf16: torch.Tensor) -> None:
 
 
 def set_attention_impl(impl: str) -> str:
-    """'auto' (tcgen05 kernels: attn_tc3.cu for 7 x 7 windows, else the two-pass kernel up to 400 tokens, else the chunked one-pass
-    kernel), 'tc1' / 'tc2' / 'tc3' (prefer that generation where it applies) or 'mma' (mma.sync kernels only); returns the previous setting."""
-    names = ["auto", "mma", "tc1", "tc2", "tc3"]
-    prev = lib().lavt_set_attention_impl(names.index(impl))
-    return names[prev] if 0 <= prev < len(names) else "auto"
+    """'auto' (attn_tc3.cu for full 7 x 7 / 12 x 12 windows, the chunked one-pass tcgen05 kernel attn_tc2.cu for every other window of
+    16+ tokens, the mma.sync kernel for smaller ones), 'tc2' (attn_tc2.cu wherever it applies) or 'tc3' (the same as auto); returns the
+    previous setting."""
+    codes = {"auto": 0, "tc2": 3, "tc3": 4}
+    if impl not in codes:
+        raise LavtError(f"attention impl must be one of {sorted(codes)}, not {impl!r}")
+    prev = lib().lavt_set_attention_impl(codes[impl])
+    return {v: k for k, v in codes.items()}.get(prev, "auto")
 
 
 def set_attention_bwd_impl(impl: str) -> str:
@@ -442,7 +445,7 @@ def set_attention_bwd_impl(impl: str) -> str:
 
 
 def window_attention_has_lse(table_t: torch.Tensor, geom: WinGeom) -> bool:
-    """True if window_attention can also write the per-row log-sum-exp for this geometry (tcgen05 kernel)."""
+    """True if window_attention can also write the per-row log-sum-exp for this geometry (tcgen05 kernels: windows of 16+ tokens)."""
     nH, L = table_t.shape
     return bool(lib().lavt_window_attention_has_lse(C.byref(geom), L, nH))
 

@@ -2,7 +2,7 @@
 // (reference WindowAttention3D.forward, lib/video_swin_transformer.py:147-165; 2-D twin lib/backbone.py:127-138)
 //     S = q k^T + relative-position bias (+ shifted-window mask)  ->  softmax  ->  O = P v       per (window, head)
 //
-// What changed against attn_tc.cu (which keeps the whole score row of <= 400 keys in TMEM and walks it twice):
+// What changed against the first generation (DESIGN.md 4.1: it kept the whole score row of <= 400 keys in TMEM and walked it twice):
 //   * the KEY axis is cut into chunks of <= 112 columns that alternate between TWO softmax warpgroups; every warpgroup owns two
 //     S buffers in TMEM, so the Q K^T of its next chunk is issued while it is still exponentiating the current one, and windows of
 //     any size (8 x 12 x 12 = 1152 keys) fit: 2 groups x 2 buffers x 112 columns + 2 x 32 accumulator columns = 512

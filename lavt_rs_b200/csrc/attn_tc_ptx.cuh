@@ -1,4 +1,4 @@
-// tcgen05 / TMEM PTX wrappers shared by the window-attention kernels (attn_tc.cu, attn_tc2.cu).
+// tcgen05 / TMEM PTX wrappers shared by the window-attention kernels (attn_tc2.cu, attn_tc3.cu, attn_bwd_tc.cu).
 #pragma once
 #include "common.cuh"
 

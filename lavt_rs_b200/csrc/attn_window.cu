@@ -1,5 +1,10 @@
-// Shifted-window attention core (reference WindowAttention3D.forward, lib/video_swin_transformer.py:147-165;
-// 2-D twin lib/backbone.py:127-138):  per (window, head)
+// Shifted-window attention forward: the one dispatch decision (window_attn_choose) and the mma.sync fallback for the
+// windows that neither tcgen05 kernel takes.  window_attn_dispatch sends every window of 16+ tokens to attn_tc3.cu (full
+// 7 x 7 / 12 x 12 windows) or attn_tc2.cu (every other window of up to 1152 tokens); what is left are clamped windows of
+// fewer than 16 tokens (e.g. stage 3 of a 32 px clip), too small for a 128-row tcgen05 tile to be worth it.
+//
+// Fallback (reference WindowAttention3D.forward, lib/video_swin_transformer.py:147-165; 2-D twin lib/backbone.py:127-138):
+// per (window, head)
 //     S = q k^T  (+ relative-position bias, + shifted-window mask)  ->  softmax  ->  O = P v
 // computed flash-style: the N x N score matrix never leaves registers.  q arrives pre-scaled by
 // head_dim^-0.5 * log2(e) (folded into the qkv GEMM epilogue) so the softmax runs in base 2 with one FADD + one
@@ -7,18 +12,13 @@
 // log2 e) through the closed form  idx(i,j) = code(i) - code(j) + const ; the -100 mask comes from per-token region
 // ids (geom.cuh) and is skipped entirely for windows that do not straddle the cyclic-shift seam -- neither the (N,N)
 // index buffer nor the (nW,N,N) mask tensor exists on the device.
-//
-// mma.sync.m16n8k16 (bf16 -> fp32).  head_dim is 32 at every Swin stage, which makes this core SIMT-issue / latency
-// bound rather than tensor bound (ncu: profiles/), so the two kernels below are organised around that:
-//   window_attn_resident_kernel  N <= 512: one CTA per (window, head) keeps the whole K and V of the head in shared
-//                                memory (loaded once with cp.async) and every warp walks 16-row query strips with NO
-//                                block-level synchronisation in the main loop; set-up cost (codes, table) is paid once
-//   window_attn_stream_kernel    larger windows (8x12x12 -> N = 1152): CTA per (q-tile, head, window), K/V tiles
-//                                streamed through a cp.async double buffer
-// Tile shapes are chosen to minimise padded work (N = 392 -> 25 strips x 5 key tiles of 80 = 400 x 400).
+// mma.sync.m16n8k16 (bf16 -> fp32), window_attn_resident_kernel: one CTA per (window, head) keeps the whole K and V of
+// the head in shared memory (loaded once with cp.async); a single warp walks the one 16-row query strip against one
+// key tile of 48.  It writes no row statistics (lse), so a training forward of such a window recomputes them in the backward.
 #include "kernels.cuh"
 
 #include <cstdlib>
+#include <cstring>
 
 namespace lavt {
 
@@ -253,86 +253,11 @@ __global__ void __launch_bounds__(256, 2) window_attn_resident_kernel(const Attn
   }
 }
 
-// ------------------------------------------------------------------------------------------------------------------
-// streamed K/V: grid (q-tiles, nH, windows), WARPS * 16 query rows per CTA
-// ------------------------------------------------------------------------------------------------------------------
-template <int WARPS, int KVT>
-__global__ void __launch_bounds__(WARPS * 32) window_attn_stream_kernel(const AttnParams p) {
-  constexpr int BQ = WARPS * 16;
-  constexpr int THREADS = WARPS * 32;
-  extern __shared__ __align__(16) uint8_t smem[];
-  const int N = p.win.N;
-  const int Npad = (N + 7) & ~7;
-  uint8_t* ks = smem;                                             // [2][KVT][64 B]
-  uint8_t* vs = ks + 2 * KVT * 64;                                // [2][KVT][64 B]
-  uint16_t* codes = reinterpret_cast<uint16_t*>(vs + 2 * KVT * 64);
-  uint8_t* rids = reinterpret_cast<uint8_t*>(codes + Npad);
-  float* tab = reinterpret_cast<float*>(rids + Npad);
-  __shared__ int s_need_mask;
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int g = lane >> 2, t = lane & 3;
-  const int q0 = blockIdx.x * BQ;
-  const int head = blockIdx.y;
-  const long long row0 = static_cast<long long>(blockIdx.z) * N;
-  const int ld = 3 * p.C;
-  const __nv_bfloat16* qbase = p.qkv + row0 * ld + head * AT_HD;
-  const __nv_bfloat16* kbase = qbase + p.C;
-  const __nv_bfloat16* vbase = qbase + 2 * p.C;
-  const bool shifted = (p.win.sd | p.win.sh | p.win.sw) != 0;
-  const int ntiles = (N + KVT - 1) / KVT;
-
-  auto load_tile = [&](int tile, int buf) {
-    for (int i = threadIdx.x; i < 2 * KVT * 4; i += THREADS) {
-      const int isv = i >= KVT * 4;
-      const int j = isv ? i - KVT * 4 : i;
-      const int r = j >> 2, c = j & 3;
-      const int key = tile * KVT + r;
-      const bool ok = key < N;
-      const __nv_bfloat16* src = (isv ? vbase : kbase) + static_cast<long long>(ok ? key : 0) * ld + c * 8;
-      cp_async_16((isv ? vs : ks) + buf * KVT * 64 + kv_off(r, c), src, ok);
-    }
-  };
-
-  if (threadIdx.x == 0) s_need_mask = 0;
-  load_tile(0, 0);
-  cp_async_commit();
-  __syncthreads();
-  setup_window(p, row0, head, N, Npad, codes, rids, tab, &s_need_mask, shifted);
-  const int rc = rel_const(p.win);
-
-  uint32_t qf[2][4];
-  const int qr0 = q0 + warp * 16 + g, qr1 = qr0 + 8;
-  const int qc0 = min(qr0, N - 1), qc1 = min(qr1, N - 1);
-  load_q_frags(qf, qbase, ld, qc0, qc1, t);
-  __syncthreads();   // codes / rids / tab / s_need_mask visible
-  const bool need_mask = s_need_mask != 0;
-  const float* tq0 = tab + (static_cast<int>(codes[qc0]) + rc);
-  const float* tq1 = tab + (static_cast<int>(codes[qc1]) + rc);
-  const int rq0 = rids[qc0], rq1 = rids[qc1];
-
-  RowState st;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) st.o[i][0] = st.o[i][1] = st.o[i][2] = st.o[i][3] = 0.f;
-  st.m0 = st.m1 = -INFINITY;
-  st.l0 = st.l1 = 0.f;
-
-  for (int tile = 0; tile < ntiles; ++tile) {
-    const int buf = tile & 1;
-    if (tile + 1 < ntiles) load_tile(tile + 1, buf ^ 1);
-    cp_async_commit();
-    cp_async_wait<1>();
-    __syncthreads();
-    attn_tile<KVT>(ks + buf * KVT * 64, vs + buf * KVT * 64, tile * KVT, N, Npad, codes, rids, tq0, tq1, rq0, rq1, need_mask, qf, st,
-                   lane);
-    __syncthreads();   // all warps done with buf before it is refilled
-  }
-  store_rows(st, p.out + row0 * p.C + head * AT_HD, p.C, qr0, qr1, N, t);
-}
 
 // ------------------------------------------------------------------------------------------------------------------
-template <int KVT>
-static int launch_resident(const AttnParams& p, long long nwin, int warps, cudaStream_t st) {
+// N < 16: one 16-row query strip, one warp, one key tile of 48
+static int launch_resident(const AttnParams& p, long long nwin, cudaStream_t st) {
+  constexpr int KVT = 48;
   const int N = p.win.N;
   const int Npad = (N + 7) & ~7;
   const int rows = ((N + KVT - 1) / KVT) * KVT;
@@ -344,41 +269,28 @@ static int launch_resident(const AttnParams& p, long long nwin, int warps, cudaS
     configured = smem;
   }
   dim3 grid(p.nH, static_cast<unsigned>(nwin));
-  kfn<<<grid, warps * 32, smem, st>>>(p);
+  kfn<<<grid, 32, smem, st>>>(p);
   LAVT_LAUNCH_CHECK("window_attn_resident_kernel");
-  return LAVT_OK;
-}
-
-template <int WARPS, int KVT>
-static int launch_stream(const AttnParams& p, long long nwin, cudaStream_t st) {
-  const int N = p.win.N;
-  const int Npad = (N + 7) & ~7;
-  const size_t smem = 4 * KVT * 64 + static_cast<size_t>(Npad) * 3 + static_cast<size_t>(p.L) * 4 + 16;
-  LAVT_REQUIRE(smem <= 200 * 1024, "attention: window too large for shared memory (N=%d, L=%d)", N, p.L);
-  auto kfn = window_attn_stream_kernel<WARPS, KVT>;
-  static size_t configured = 0;
-  if (smem > configured) {
-    LAVT_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-    configured = smem;
-  }
-  constexpr int BQ = WARPS * 16;
-  dim3 grid((N + BQ - 1) / BQ, p.nH, static_cast<unsigned>(nwin));
-  kfn<<<grid, WARPS * 32, smem, st>>>(p);
-  LAVT_LAUNCH_CHECK("window_attn_stream_kernel");
   return LAVT_OK;
 }
 
 int attn_impl_setting(int set) {
   static int impl = -1;
   if (impl < 0) {
-    const char* e = getenv("LAVT_ATTN_IMPL");
-    // default: auto (tcgen05 kernels where they apply); "mma" = mma.sync only, "tc1" / "tc2" = prefer the first / second generation
-    impl = !e ? 0 : e[0] == 'm' ? 1 : (e[0] == 't' && e[1] == 'c' && e[2] == '1') ? 2 : (e[0] == 't' && e[1] == 'c' && e[2] == '2') ? 3 :
-           (e[0] == 't' && e[1] == 'c' && e[2] == '3') ? 4 : 0;
+    const char* e = getenv("LAVT_ATTN_IMPL");      // A/B runs: "tc2" / "tc3"; anything else is auto
+    impl = e && !strcmp(e, "tc2") ? 3 : e && !strcmp(e, "tc3") ? 4 : 0;
   }
   const int prev = impl;
-  if (set >= 0) impl = set <= 4 ? set : 0;
+  if (set >= 0) impl = set;
   return prev;
+}
+
+AttnKernel window_attn_choose(const AttnParams& p) {
+  // tc3 is the faster kernel wherever it applies (stage 2 of the bench at N = 392: 203 vs 331 us, DESIGN 4.1); forcing tc2 is for A/B runs
+  if (attn_impl_setting(-1) == 3 && window_attn_tc2_supported(p)) return AttnKernel::TC2;
+  if (window_attn_tc3_supported(p)) return AttnKernel::TC3;
+  if (window_attn_tc2_supported(p)) return AttnKernel::TC2;
+  return AttnKernel::MMA;
 }
 
 int window_attn_dispatch(const AttnParams& p, cudaStream_t st) {
@@ -390,53 +302,14 @@ int window_attn_dispatch(const AttnParams& p, cudaStream_t st) {
   LAVT_REQUIRE(g.N <= g.Wd * g.Wh * g.Ww, "attention: effective window larger than configured window");
   const long long nwin = 1LL * g.B * g.nwd * g.nwh * g.nww;
   LAVT_REQUIRE(nwin > 0 && nwin < 65536, "attention: window count %lld out of range", nwin);
-  const int N = g.N;
-  {
-    // LAVT_ATTN_IMPL=mma (or lavt_set_attention_impl(1)) forces the mma.sync kernels below
-    const int impl = attn_impl_setting(-1);
-    if (impl != 1) {
-      // auto: the resident two-pass kernel (attn_tc.cu) for windows of <= 400 tokens, where it is still the faster one (7.1 vs 8.0 ms
-      // per 8-clip step), the key-chunked one-pass kernel (attn_tc2.cu) for everything larger (8 x 12 x 12: 14.9 ms vs 21.8 ms for the
-      // mma.sync kernels); "tc2" forces the chunked kernel everywhere
-      if (impl == 3 && window_attn_tc2_supported(p)) return window_attn_tc2_dispatch(p, st);
-      // 7 x 7 windows: the row-parallel kernel with vector bias loads (attn_tc3.cu); "tc1" / "tc2" keep the older generations for A/B runs
-      if ((impl == 0 || impl == 4) && window_attn_tc3_supported(p)) return window_attn_tc3_dispatch(p, st);
-      if (window_attn_tc_supported(p)) return window_attn_tc_dispatch(p, st);
-      if (window_attn_tc2_supported(p)) return window_attn_tc2_dispatch(p, st);
-    }
+  switch (window_attn_choose(p)) {
+    case AttnKernel::TC3: return window_attn_tc3_dispatch(p, st);
+    case AttnKernel::TC2: return window_attn_tc2_dispatch(p, st);
+    case AttnKernel::MMA: break;
   }
-  LAVT_REQUIRE(p.lse == nullptr, "attention: row statistics (lse) are produced by the tcgen05 kernel only (N=%d)", N);
-  if (N <= 512) {
-    // key tile = the candidate with the least padding; warps = a divisor-friendly count of the 16-row strips
-    const int kvts[3] = {80, 64, 48};
-    int best = 0, best_pad = 1 << 30;
-    for (int i = 0; i < 3; ++i) {
-      const int pad = ((N + kvts[i] - 1) / kvts[i]) * kvts[i];
-      if (pad < best_pad) { best_pad = pad; best = i; }
-    }
-    const int strips = (N + 15) / 16;
-    int warps = strips < 8 ? strips : 8;
-    for (int w = 8; w >= 4; --w) {
-      if (strips % w == 0) { warps = w; break; }
-    }
-    if (strips >= 8 && strips % warps != 0) warps = 6;
-    static int env_kvt = -1, env_warps = -1;
-    if (env_kvt < 0) {
-      const char* e1 = getenv("LAVT_ATTN_KVT");
-      const char* e2 = getenv("LAVT_ATTN_WARPS");
-      env_kvt = e1 ? atoi(e1) : 0;
-      env_warps = e2 ? atoi(e2) : 0;
-    }
-    if (env_kvt == 80) best = 0; else if (env_kvt == 64) best = 1; else if (env_kvt == 48) best = 2;
-    if (env_warps > 0) warps = env_warps;
-    switch (best) {
-      case 0: return launch_resident<80>(p, nwin, warps, st);
-      case 1: return launch_resident<64>(p, nwin, warps, st);
-      default: return launch_resident<48>(p, nwin, warps, st);
-    }
-  }
-  if (N % 128 == 0 || N > 1024) return launch_stream<8, 64>(p, nwin, st);
-  return launch_stream<4, 64>(p, nwin, st);
+  LAVT_REQUIRE(g.N < 16, "attention: no kernel takes a window of %d tokens (tcgen05: 16 ... 1152, mma.sync fallback: < 16)", g.N);
+  LAVT_REQUIRE(p.lse == nullptr, "attention: row statistics (lse) are produced by the tcgen05 kernels only (N=%d)", g.N);
+  return launch_resident(p, nwin, st);
 }
 
 }  // namespace lavt

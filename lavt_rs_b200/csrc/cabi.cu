@@ -187,11 +187,11 @@ int lavt_window_attention_has_lse(const lavt_win_geom_t* geom, int32_t L, int32_
   std::memset(&p, 0, sizeof(p));
   std::memcpy(&p.win, geom, sizeof(WinGeom));
   p.nH = nH; p.C = nH * 32; p.L = L;
-  return (attn_impl_setting(-1) != 1 && (window_attn_tc_supported(p) || window_attn_tc2_supported(p))) ? 1 : 0;
+  return window_attn_choose(p) != AttnKernel::MMA ? 1 : 0;
 }
 
 int lavt_set_attention_bwd_impl(int32_t impl) { return attn_bwd_impl_setting(impl >= 0 && impl <= 2 ? impl : 0); }
-int lavt_set_attention_impl(int32_t impl) { return attn_impl_setting(impl >= 0 && impl <= 4 ? impl : 0); }
+int lavt_set_attention_impl(int32_t impl) { return attn_impl_setting(impl == 3 || impl == 4 ? impl : 0); }
 
 int64_t lavt_instnorm_workspace_floats(int32_t B, int64_t n, int32_t C) { return colstats_workspace_floats(B, n, C); }
 

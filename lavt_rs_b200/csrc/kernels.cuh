@@ -39,10 +39,11 @@ struct AttnParams {
   float* lse;                 // [rows, nH] log2-sum-exp2 of every score row, or nullptr (training: saved for the backward; tcgen05 kernel only)
 };
 int window_attn_dispatch(const AttnParams& p, cudaStream_t st);
-// tcgen05 / TMEM variant (attn_tc.cu): windows of up to 400 tokens
-int attn_impl_setting(int set);   // set < 0: query only; returns the previous value (0 = auto, 1 = mma.sync only, 2 = prefer attn_tc.cu, 3 = attn_tc2.cu, 4 = attn_tc3.cu)
-bool window_attn_tc_supported(const AttnParams& p);
-int window_attn_tc_dispatch(const AttnParams& p, cudaStream_t st);
+int attn_impl_setting(int set);   // set < 0: query only; returns the previous value (0 = auto, 3 = prefer attn_tc2.cu, 4 = attn_tc3.cu where it applies = auto)
+// The kernel window_attn_dispatch runs for p (host arithmetic only, no device call): attn_tc3.cu, attn_tc2.cu or the mma.sync
+// fallback of attn_window.cu (windows of fewer than 16 tokens; the only choice that writes no lse)
+enum class AttnKernel { TC3, TC2, MMA };
+AttnKernel window_attn_choose(const AttnParams& p);
 // second generation (attn_tc2.cu): key-chunked, one-pass softmax, windows of up to 1152 tokens
 bool window_attn_tc2_supported(const AttnParams& p);
 int window_attn_tc2_dispatch(const AttnParams& p, cudaStream_t st);

@@ -38,12 +38,22 @@ CASES = [  # (B, D, H, W), window, shifted, heads
     # attn_tc3.cu corner cases: a two-frame window (N = 98, one partial tile), a single (window, head) unit, and enough units per CTA that the
     # K / V stages, the Q ring and the bias table (several heads per CTA) all wrap around
     ((1, 2, 14, 14), (8, 7, 7), True, 4), ((1, 8, 7, 7), (8, 7, 7), False, 1), ((4, 8, 24, 24), (8, 7, 7), True, 16),
+    # clamped windows of fewer than 16 tokens (mma.sync fallback): N = 4, 8, 6, a single token, the 12 x 12 table, N = 14 shifted along h
+    ((1, 4, 1, 1), (8, 7, 7), True, 4), ((1, 8, 1, 1), (8, 7, 7), True, 8), ((2, 3, 1, 2), (8, 7, 7), True, 32),
+    ((1, 1, 1, 1), (8, 7, 7), False, 4), ((2, 2, 2, 3), (8, 12, 12), True, 16), ((1, 1, 14, 2), (8, 7, 7), True, 4),
+    # the smallest attn_tc2.cu windows (N = 16 shifted along d, 30)
+    ((1, 16, 2, 1), (8, 7, 7), True, 4), ((2, 2, 3, 5), (8, 7, 7), True, 8),
+    # clamped windows of 48 ... 400 tokens: stage 3 of the video models at 8 x 192^2 (w7, N = 288), 8 x 160^2 (w7 and w12, N = 200) and
+    # 4 x 320^2 (w12, N = 400), shorter clips, and a window clamped along w only (shift and mask along h)
+    ((1, 8, 6, 6), (8, 7, 7), True, 32), ((2, 8, 5, 5), (8, 7, 7), True, 32), ((1, 4, 6, 6), (8, 7, 7), True, 16),
+    ((1, 8, 3, 3), (8, 7, 7), True, 8), ((1, 8, 14, 5), (8, 7, 7), True, 4), ((1, 8, 5, 5), (8, 12, 12), True, 32),
+    ((1, 4, 10, 10), (8, 12, 12), True, 32),
 ]
 
 
-# auto = attn_tc3.cu for 7 x 7 windows (row-parallel warpgroups, run-padded keys), else tc1 / tc2; tc2 = one-pass chunked tcgen05 kernel
-# (every N); tc1 = two-pass tcgen05 kernel where it applies (N <= 400); mma = mma.sync
-@pytest.mark.parametrize("impl", ["auto", "tc1", "tc2", "mma"])
+# auto = attn_tc3.cu for full 7 x 7 / 12 x 12 windows (row-parallel warpgroups, run-padded keys), attn_tc2.cu for the other windows of 16+
+# tokens, the mma.sync kernel below that; tc2 = the one-pass chunked tcgen05 kernel wherever it applies (N >= 16)
+@pytest.mark.parametrize("impl", ["auto", "tc2"])
 @pytest.mark.parametrize("dims,window,shifted,nH", CASES)
 def test_window_attention_matches_torch(dims, window, shifted, nH, impl):
     from lavt_rs_b200 import _cabi as K
@@ -108,7 +118,7 @@ def test_one_pass_softmax_slow_path(dims, window, nH, pattern, impl):
     table = torch.randn(L, nH, device="cuda", generator=g)
     out = torch.empty(rows, C, device="cuda", dtype=torch.bfloat16)
     lse = torch.empty(rows, nH, device="cuda", dtype=torch.float32)
-    prev = K.set_attention_impl(impl)       # tc3 falls through to the other generations for windows that are not 7 x 7
+    prev = K.set_attention_impl(impl)       # tc3 = auto: attn_tc2.cu for the windows that are not full 7 x 7 / 12 x 12
     try:
         K.window_attention(qkv, table.t().contiguous(), geom, out, lse=lse)
         torch.cuda.synchronize()

@@ -1,4 +1,4 @@
-"""Attention-kernel micro-benchmark at the bench shapes (8 clips): python tools/bench_attn.py [impl ...]   (impl: auto tc1 tc2 mma)"""
+"""Attention-kernel micro-benchmark at the bench shapes (8 clips): python tools/bench_attn.py [impl ...]   (impl: auto tc2 tc3)"""
 import math, os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from lavt_rs_b200 import _cabi as K

@@ -8,7 +8,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LIB = os.path.join(ROOT, "lavt_rs_b200", "_lib", "liblavt_b200.so")
-KERNELS = ("gemm_bf16_tc_kernel", "window_attn_tc_kernel", "window_attn_tc2_kernel", "window_attn_tc3_kernel", "window_attn_bwd_tc_kernel", "window_attn_bwd_kernel", "window_attn_resident_kernel",
+KERNELS = ("gemm_bf16_tc_kernel", "window_attn_tc2_kernel", "window_attn_tc3_kernel", "window_attn_bwd_tc_kernel", "window_attn_bwd_kernel", "window_attn_resident_kernel",
            "pwam_core")
 out = subprocess.run(["cuobjdump", "-sass", LIB], capture_output=True, text=True).stdout
 name, stats, first = None, collections.OrderedDict(), {}
