@@ -230,6 +230,12 @@ int lavt_gate_transpose(const float* x, int64_t ldx, const float* gate, int64_t 
  * C2 = 0 (skip NULL) is a plain upsample: nn.Upsample(scale_factor=2, bilinear, align_corners=True) of lib/vlt.py:48,75,437-452 */
 int lavt_upsample_concat(const void* prev_bf16, int32_t ph, int32_t pw, int32_t C1, const void* skip_bf16, int32_t C2,
                          void* out_bf16, int32_t n_img, int32_t H, int32_t W, void* stream);
+/* conv3x3 + folded BN + ReLU of cat[bilinear(Y [n,h,w,C_Y] -> HxW, align_corners=True), skip], evaluated on the coarse grid:
+ * out bf16 [n,H,W,hid] = ReLU(addend + s[co] * sum_tap sum_corner beta * Z[n, corner, tap*hid + co]), Z bf16 [n,h,w,9*hid] = Y . W_tap
+ * (row tap*hid + co of the weight holds w[co, :C_Y, ky, kx], tap = ky*3+kx; zero padding on the fine grid).  addend = P fp32 [n,H,W,hid]
+ * (the skip half of the conv with the BN folded in) or, with P NULL, b fp32 [hid]. */
+int lavt_upconv_blend(const void* z_bf16, int32_t h, int32_t w, int32_t hid, const float* P, const float* s, const float* b, void* out_bf16,
+                      int32_t n_img, int32_t H, int32_t W, void* stream);
 /* conv1_1: logits[pix, 0:2] = y[pix, :] . w[0:2, :] + b */
 int lavt_conv1x1_logits(const void* y_bf16, const float* w, const float* b, float* out, int64_t npix, int32_t C, void* stream);
 /* (n,h,w,2) fp32 -> (n,2,H,W) fp32 NCHW, bilinear align_corners=True */

@@ -100,6 +100,7 @@ SIGNATURES = {
     "lavt_split3_bf16": [_vp, _i64, _vp, _i64, _i32, _vp],
     "lavt_bert_attention_f32": [_vp, _vp, _vp, _i32, _i32, _i32, _i32, _vp],
     "lavt_upsample_concat": [_vp, _i32, _i32, _i32, _vp, _i32, _vp, _i32, _i32, _i32, _vp],
+    "lavt_upconv_blend": [_vp, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _i32, _i32, _i32, _vp],
     "lavt_conv1x1_logits": [_vp, _vp, _vp, _vp, _i64, _i32, _vp],
     "lavt_upsample_logits": [_vp, _vp, _i32, _i32, _i32, _i32, _i32, _vp],
     "lavt_nhwc_to_nchw": [_vp, _vp, _i32, _i32, _i32, _vp],
@@ -582,6 +583,21 @@ def upsample_concat(prev, skip, out) -> None:
     check(lib().lavt_upsample_concat(prev.data_ptr(), ph, pw, C1, skip.data_ptr(), C2,
                                      _c(out, torch.bfloat16, "out").data_ptr(), n, H, W, stream_ptr()),
           "lavt_upsample_concat")
+
+
+def upconv_blend(z, p, s, b, out) -> None:
+    """z bf16 [n,h,w,9*hid] (Z = Y . W_tap on the coarse map); p fp32 [n,H,W,hid] or None; s, b fp32 [hid]; out bf16 [n,H,W,hid]
+    = ReLU((p if given, else b) + s * conv3x3 of the bilinear (align_corners) upsample, assembled from z)."""
+    n, h, w, c9 = _c(z, torch.bfloat16, "z").shape
+    n2, H, W, hid = _c(out, torch.bfloat16, "out").shape
+    if n != n2 or c9 != 9 * hid or tuple(s.shape) != (hid,) or tuple(b.shape) != (hid,) or (p is not None and tuple(p.shape) != (n, H, W, hid)):
+        raise LavtError("upconv_blend: shape mismatch")
+    t0 = TIMER.begin()
+    check(lib().lavt_upconv_blend(z.data_ptr(), h, w, hid, None if p is None else _c(p, torch.float32, "p").data_ptr(),
+                                  _c(s, torch.float32, "s").data_ptr(), _c(b, torch.float32, "b").data_ptr(), out.data_ptr(),
+                                  n, H, W, stream_ptr()), "lavt_upconv_blend")
+    TIMER.end(t0, "upconv_blend_kernel", 2.0 * 36 * n * H * W * hid, 2.0 * z.numel() + 2.0 * out.numel() + (4.0 * p.numel() if p is not None else 0.0),
+              f"{n}x{h}x{w} -> {H}x{W} hid{hid}")
 
 
 def conv1x1_logits(y, w, b, out) -> None:

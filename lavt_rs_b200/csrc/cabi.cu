@@ -250,6 +250,11 @@ int lavt_upsample_concat(const void* prev_bf16, int32_t ph, int32_t pw, int32_t 
   return upsample_concat_dispatch(CB(prev_bf16), ph, pw, C1, CB(skip_bf16), C2, MB(out_bf16), n_img, H, W, S(stream));
 }
 
+int lavt_upconv_blend(const void* z_bf16, int32_t h, int32_t w, int32_t hid, const float* P, const float* s, const float* b, void* out_bf16,
+                      int32_t n_img, int32_t H, int32_t W, void* stream) {
+  return upconv_blend_dispatch(CB(z_bf16), h, w, hid, P, s, b, MB(out_bf16), n_img, H, W, S(stream));
+}
+
 int lavt_conv1x1_logits(const void* y_bf16, const float* w, const float* b, float* out, int64_t npix, int32_t C, void* stream) {
   return conv1x1_logits_dispatch(CB(y_bf16), w, b, out, npix, C, S(stream));
 }

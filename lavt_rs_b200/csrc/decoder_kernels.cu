@@ -163,6 +163,188 @@ int upsample_concat_dispatch(const __nv_bfloat16* prev, int ph, int pw, int C1, 
   return LAVT_OK;
 }
 
+// ---- conv3x3 of a bilinear upsample, evaluated on the coarse grid ----
+// conv3x3(up(Y))[p] = sum_tap [p + tap inside H x W] sum_corner beta(p + tap, corner) * Z[corner, tap], Z = W_tap . Y (one GEMM on the
+// coarse map).  The blend below finishes a decoder conv+BN+ReLU: out = ReLU(addend + s * that sum), addend = the skip half of the conv
+// with the BN folded in (P, fp32) or, without a skip, the folded BN shift b.
+__device__ __forceinline__ void blend_epilogue(const float* acc, const float* __restrict__ P, const float* __restrict__ s,
+                                               const float* __restrict__ b, long long pix, int hid, int c, __nv_bfloat16* __restrict__ out) {
+  const float4 s0 = __ldg(reinterpret_cast<const float4*>(s + c)), s1 = __ldg(reinterpret_cast<const float4*>(s + c + 4));
+  const float* add = P ? P + pix * hid + c : b + c;
+  const float4 a0 = __ldg(reinterpret_cast<const float4*>(add)), a1 = __ldg(reinterpret_cast<const float4*>(add + 4));
+  const float sv[8] = {s0.x, s0.y, s0.z, s0.w, s1.x, s1.y, s1.z, s1.w}, av[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
+  uint32_t o[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k)
+    o[k] = pack_bf16x2(fmaxf(fmaf(sv[2 * k], acc[2 * k], av[2 * k]), 0.f), fmaxf(fmaf(sv[2 * k + 1], acc[2 * k + 1], av[2 * k + 1]), 0.f));
+  *reinterpret_cast<uint4*>(out + pix * hid + c) = make_uint4(o[0], o[1], o[2], o[3]);
+}
+
+// any (h, w) -> (H, W): thread per (fine pixel, 8 channels), the 9 x 4 (tap, corner) terms read straight from Z
+__global__ void __launch_bounds__(256) upconv_blend_kernel(const __nv_bfloat16* __restrict__ Z, int h, int w, int hid,
+                                                           const float* __restrict__ P, const float* __restrict__ s,
+                                                           const float* __restrict__ b, __nv_bfloat16* __restrict__ out, int H, int W) {
+  const int g8 = hid / 8;
+  const int xi = blockIdx.x * blockDim.x + threadIdx.x;
+  if (xi >= W * g8) return;
+  const int x = xi / g8;
+  const int c = (xi - x * g8) * 8;
+  const int y = blockIdx.y;
+  const long long img = blockIdx.z;
+  const long long ldz = 9LL * hid;
+  const __nv_bfloat16* zimg = Z + img * h * w * ldz + c;
+  float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  for (int ky = 0; ky < 3; ++ky) {
+    const int qy = y + ky - 1;
+    if (qy < 0 || qy >= H) continue;              // zero padding of the fine image
+    int y0, y1;
+    float fy;
+    bilinear_taps(qy, h, H, y0, y1, fy);
+    for (int kx = 0; kx < 3; ++kx) {
+      const int qx = x + kx - 1;
+      if (qx < 0 || qx >= W) continue;
+      int x0, x1;
+      float fx;
+      bilinear_taps(qx, w, W, x0, x1, fx);
+      const float w00 = (1.f - fy) * (1.f - fx), w01 = (1.f - fy) * fx, w10 = fy * (1.f - fx), w11 = fy * fx;
+      const __nv_bfloat16* zt = zimg + (ky * 3 + kx) * hid;
+      const uint4 a = __ldg(reinterpret_cast<const uint4*>(zt + (static_cast<long long>(y0) * w + x0) * ldz));
+      const uint4 bq = __ldg(reinterpret_cast<const uint4*>(zt + (static_cast<long long>(y0) * w + x1) * ldz));
+      const uint4 cc = __ldg(reinterpret_cast<const uint4*>(zt + (static_cast<long long>(y1) * w + x0) * ldz));
+      const uint4 d = __ldg(reinterpret_cast<const uint4*>(zt + (static_cast<long long>(y1) * w + x1) * ldz));
+      const uint32_t ua[4] = {a.x, a.y, a.z, a.w}, ub[4] = {bq.x, bq.y, bq.z, bq.w}, uc[4] = {cc.x, cc.y, cc.z, cc.w},
+                     ud[4] = {d.x, d.y, d.z, d.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 fa = unpack_bf16x2(ua[j]), fb = unpack_bf16x2(ub[j]), fc = unpack_bf16x2(uc[j]), fd = unpack_bf16x2(ud[j]);
+        acc[2 * j] += w00 * fa.x + w01 * fb.x + w10 * fc.x + w11 * fd.x;
+        acc[2 * j + 1] += w00 * fa.y + w01 * fb.y + w10 * fc.y + w11 * fd.y;
+      }
+    }
+  }
+  blend_epilogue(acc, P, s, b, (img * H + y) * W + x, hid, c, out);
+}
+
+// Exact x2 (H == 2h, W == 2w: every SimpleDecoding level).  A block stages the Z rows of a UB_TI x UB_TJ coarse tile plus a one-pixel
+// border (all 9 taps, UB_CC channels) in shared memory; a thread owns the 2 x 2 fine pixels above coarse pixel (i, j) for 8 channels.
+// Their 9 taps x 4 corners touch 7 x 7 of the 9 x 9 (window pixel, tap) entries of the 3 x 3 window (i-1 .. i+1, j-1 .. j+1): 49 shared
+// loads for 4 outputs instead of 144.  Fine row q = 2i - 1 + u (u = 0..3) interpolates window rows (0, 1) for u < 2 and (1, 2) otherwise;
+// its fraction is taken against that fixed pair and clamped, as in upsample2x_concat_kernel, so the clamped window at the map border
+// (weight 0 or an identical row) gives the same value.  Accumulation in packed fp32x2.
+constexpr int UB_TI = 4, UB_TJ = 8, UB_CC = 32;
+constexpr int UB_THREADS = UB_TI * UB_TJ * (UB_CC / 8);
+constexpr int UB_G = UB_CC / 8;
+static_assert(UB_G == 4, "the addend prefetch gives each of a coarse pixel's 4 channel groups one of its 4 fine pixels");
+__global__ void __launch_bounds__(UB_THREADS) upconv2x_blend_kernel(const __nv_bfloat16* __restrict__ Z, int h, int w, int hid,
+                                                                    const float* __restrict__ P, const float* __restrict__ s,
+                                                                    const float* __restrict__ b, __nv_bfloat16* __restrict__ out) {
+  __shared__ uint4 zs[(UB_TI + 2) * (UB_TJ + 2) * 9 * UB_G];        // [window row][window col][tap][8-channel group]
+  const int H = 2 * h, W = 2 * w;
+  const int cgroups = hid / UB_CC;
+  const int jt = blockIdx.x / cgroups;
+  const int c0 = (blockIdx.x - jt * cgroups) * UB_CC;
+  const int i0 = blockIdx.y * UB_TI, j0 = jt * UB_TJ;
+  const long long img = blockIdx.z;
+  const long long ldz = 9LL * hid;
+  const __nv_bfloat16* zimg = Z + img * h * w * ldz + c0;
+  const int g = threadIdx.x % UB_G, tj = (threadIdx.x / UB_G) % UB_TJ, ti = threadIdx.x / (UB_G * UB_TJ);
+  const int i = i0 + ti, j = j0 + tj;
+  // the UB_G threads of a coarse pixel read its 4 fine pixels' addend rows (UB_CC fp32 = one 128-byte line each) in the epilogue:
+  // start pulling them into L2 now, so that those loads do not wait on HBM after the blend
+  if (P != nullptr && i < h && j < w)
+    asm volatile("prefetch.global.L2 [%0];" ::"l"(P + ((img * H + 2 * i + (g >> 1)) * W + 2 * j + (g & 1)) * hid + c0));
+  // asynchronous copies: every thread has all of its staging loads in flight at once
+  for (int e = threadIdx.x; e < (UB_TI + 2) * (UB_TJ + 2) * 9 * UB_G; e += UB_THREADS) {
+    const int ge = e % UB_G;
+    int r = e / UB_G;
+    const int tap = r % 9;
+    r /= 9;
+    const int wc = r % (UB_TJ + 2), wr = r / (UB_TJ + 2);
+    const int ci = min(max(i0 - 1 + wr, 0), h - 1), cj = min(max(j0 - 1 + wc, 0), w - 1);
+    cp_async_16(&zs[e], zimg + (static_cast<long long>(ci) * w + cj) * ldz + tap * hid + ge * 8, true);
+  }
+  cp_async_commit();
+  cp_async_wait<0>();
+  __syncthreads();
+  if (i >= h || j >= w) return;
+  const float sy = (H > 1) ? static_cast<float>(h - 1) / static_cast<float>(H - 1) : 0.f;
+  const float sx = (W > 1) ? static_cast<float>(w - 1) / static_cast<float>(W - 1) : 0.f;
+  float ylo[4], yhi[4], xlo[4], xhi[4];         // weights of the lower / upper row (column) of the pair; 0 outside the fine image
+#pragma unroll
+  for (int u = 0; u < 4; ++u) {
+    const int qy = 2 * i - 1 + u, qx = 2 * j - 1 + u;
+    const float fy = fminf(fmaxf(static_cast<float>(qy) * sy - static_cast<float>(u < 2 ? i - 1 : i), 0.f), 1.f);
+    const float fx = fminf(fmaxf(static_cast<float>(qx) * sx - static_cast<float>(u < 2 ? j - 1 : j), 0.f), 1.f);
+    const bool vy = qy >= 0 && qy < H, vx = qx >= 0 && qx < W;
+    ylo[u] = vy ? 1.f - fy : 0.f;
+    yhi[u] = vy ? fy : 0.f;
+    xlo[u] = vx ? 1.f - fx : 0.f;
+    xhi[u] = vx ? fx : 0.f;
+  }
+  uint64_t acc[4][4];                           // [fine pixel a * 2 + b][channel pair]
+#pragma unroll
+  for (int o = 0; o < 4; ++o)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) acc[o][k] = 0;
+  const uint4* zb = zs + (ti * (UB_TJ + 2) + tj) * 9 * UB_G + g;
+#pragma unroll
+  for (int ky = 0; ky < 3; ++ky)
+#pragma unroll
+    for (int kx = 0; kx < 3; ++kx)
+#pragma unroll
+      for (int wr = 0; wr < 3; ++wr)
+#pragma unroll
+        for (int wc = 0; wc < 3; ++wc) {
+          // window rows used by this tap: ky + a for a in {0, 1}, pair base (ky + a >= 2)
+          if (wr < (ky >= 2 ? 1 : 0) || wr > (ky >= 1 ? 2 : 1) || wc < (kx >= 2 ? 1 : 0) || wc > (kx >= 1 ? 2 : 1)) continue;
+          const uint4 v = zb[((wr * (UB_TJ + 2) + wc) * 9 + ky * 3 + kx) * UB_G];
+          const uint32_t uv[4] = {v.x, v.y, v.z, v.w};
+          uint64_t f[4];
+#pragma unroll
+          for (int k = 0; k < 4; ++k) f[k] = up_pk2(__uint_as_float(uv[k] << 16), __uint_as_float(uv[k] & 0xffff0000u));
+#pragma unroll
+          for (int a = 0; a < 2; ++a)
+#pragma unroll
+            for (int bb = 0; bb < 2; ++bb) {
+              const int u = ky + a, x = kx + bb, rb = u >= 2 ? 1 : 0, cb = x >= 2 ? 1 : 0;
+              if (wr != rb && wr != rb + 1) continue;
+              if (wc != cb && wc != cb + 1) continue;
+              const float wt = (wr == rb ? ylo[u] : yhi[u]) * (wc == cb ? xlo[x] : xhi[x]);
+              const uint64_t W2 = up_pk2(wt, wt);
+#pragma unroll
+              for (int k = 0; k < 4; ++k) asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[a * 2 + bb][k]) : "l"(W2), "l"(f[k]));
+            }
+        }
+  const int c = c0 + g * 8;
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int bb = 0; bb < 2; ++bb) {
+      float av[8];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) asm("mov.b64 {%0, %1}, %2;" : "=f"(av[2 * k]), "=f"(av[2 * k + 1]) : "l"(acc[a * 2 + bb][k]));
+      blend_epilogue(av, P, s, b, (img * H + 2 * i + a) * W + 2 * j + bb, hid, c, out);
+    }
+}
+
+int upconv_blend_dispatch(const __nv_bfloat16* Z, int h, int w, int hid, const float* P, const float* s, const float* b,
+                          __nv_bfloat16* out, int n_img, int H, int W, cudaStream_t st) {
+  LAVT_REQUIRE(hid % 8 == 0 && hid > 0 && s != nullptr && (P != nullptr || b != nullptr), "upconv_blend: hid must be a multiple of 8; s and P or b required");
+  LAVT_REQUIRE(h <= H && w <= W && h > 0 && w > 0, "upconv_blend: coarse map (%dx%d) larger than the output (%dx%d)", h, w, H, W);
+  LAVT_REQUIRE(n_img > 0 && n_img < 65536 && H > 0 && H < 65536 && W > 0, "upconv_blend: empty or too large input");
+  if (H == 2 * h && W == 2 * w && hid % UB_CC == 0) {
+    const long long gx = static_cast<long long>((w + UB_TJ - 1) / UB_TJ) * (hid / UB_CC);
+    LAVT_REQUIRE(gx < (1LL << 31), "upconv_blend: map too wide");
+    upconv2x_blend_kernel<<<dim3(static_cast<unsigned>(gx), (h + UB_TI - 1) / UB_TI, n_img), UB_THREADS, 0, st>>>(Z, h, w, hid, P, s, b, out);
+    LAVT_LAUNCH_CHECK("upconv2x_blend_kernel");
+    return LAVT_OK;
+  }
+  const int per_row = W * (hid / 8);
+  upconv_blend_kernel<<<dim3((per_row + 255) / 256, H, n_img), 256, 0, st>>>(Z, h, w, hid, P, s, b, out, H, W);
+  LAVT_LAUNCH_CHECK("upconv_blend_kernel");
+  return LAVT_OK;
+}
+
 // 8 lanes per pixel (4 pixels per warp): logits[pix, o] = sum_c y[pix, c] * w[o, c] + b[o], o in {0, 1}; w staged in smem
 __global__ void __launch_bounds__(256) conv1x1_logits_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ w,
                                                              const float* __restrict__ b, float* __restrict__ out, long long npix,

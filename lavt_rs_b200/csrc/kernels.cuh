@@ -146,6 +146,8 @@ int rows_to_cf_dispatch(const float* in, float* out, int B, int Nl, int C, cudaS
 
 int upsample_concat_dispatch(const __nv_bfloat16* prev, int ph, int pw, int C1, const __nv_bfloat16* skip, int C2,
                              __nv_bfloat16* out, int n_img, int H, int W, cudaStream_t st);
+int upconv_blend_dispatch(const __nv_bfloat16* Z, int h, int w, int hid, const float* P, const float* s, const float* b,
+                          __nv_bfloat16* out, int n_img, int H, int W, cudaStream_t st);
 int conv1x1_logits_dispatch(const __nv_bfloat16* y, const float* w, const float* b, float* out, long long npix, int C,
                             cudaStream_t st);
 int upsample_logits_dispatch(const float* in, float* out, int n_img, int h, int w, int H, int W, cudaStream_t st);

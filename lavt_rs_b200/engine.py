@@ -603,6 +603,34 @@ def _conv_taps(conv) -> torch.Tensor:
     return w.permute(0, 2, 3, 1).reshape(w.shape[0], -1).to(torch.bfloat16).contiguous()   # [(ky*3+kx)*Cin + ci]
 
 
+def _upconv_bn_relu(y: torch.Tensor, skip: Optional[torch.Tensor], dec, conv_name: str, bn_name: str, ws: Workspace,
+                    out: torch.Tensor) -> None:
+    """out = ReLU(BN(conv3x3(cat[bilinear(y -> out size, align_corners=True), skip]))) without the upsampled map: conv and upsample are
+    both linear, so the upsampled half of the conv is Z = W_tap . y on the coarse grid (one GEMM, N = 9 * hid) blended by
+    upconv_blend.  At the x2 levels that is a quarter of the FLOPs of the conv over up(y).  ``skip`` None: no skip channels."""
+    conv, bn = getattr(dec, conv_name), getattr(dec, bn_name)
+    if bn.training:
+        raise K.LavtError("SimpleDecoding on the B200 path is inference-only (BatchNorm must be in eval mode)")
+    n_img, h, w, cy = y.shape
+    _, H, W, hid = out.shape
+    dev = y.device
+    # row tap*hid + co holds w[co, :C_Y, ky, kx]
+    wy = dec.prepared.get(conv_name + "_up", [conv.weight],
+                          lambda: conv.weight.detach()[:, :cy].permute(2, 3, 0, 1).reshape(9 * hid, cy).to(torch.bfloat16).contiguous())
+    s, b = dec.prepared.get(bn_name, [bn.weight, bn.bias, bn.running_mean, bn.running_var], lambda: _bn_fold(bn))
+    z = ws.get("dec_z", (n_img, h, w, 9 * hid), torch.bfloat16, dev)
+    K.gemm_bf16(y.view(-1, cy), wy, out_bf16=z.view(-1, 9 * hid))
+    p = None
+    if skip is not None:
+        w_s = dec.prepared.get(conv_name + "_skip", [conv.weight],
+                               lambda: conv.weight.detach()[:, cy:].permute(0, 2, 3, 1).reshape(hid, -1).to(torch.bfloat16).contiguous())
+        p = ws.get("dec_p", (n_img, H, W, hid), torch.float32, dev)
+        K.conv3x3_bf16(skip, w_s, cscale=s, bias=b, out_f32=p.view(-1, hid))
+        _count(1)
+    K.upconv_blend(z, p, s, b, out)
+    _count(2)
+
+
 def _cbr(x_nhwc: torch.Tensor, dec, conv_name: str, bn_name: str, out: torch.Tensor) -> None:
     conv, bn = getattr(dec, conv_name), getattr(dec, bn_name)
     if bn.training:
@@ -633,27 +661,22 @@ def decoder_nhwc(dec, c4: torch.Tensor, c3: torch.Tensor, c2: torch.Tensor, c1: 
         _, H, W, Cs = skip.shape
         if y.shape[1] > H or y.shape[2] > W:
             raise K.LavtError("decoder: coarser map is larger than the skip connection")
-        cat = ws.get("dec_cat", (n_img, H, W, y.shape[-1] + Cs), torch.bfloat16, dev)
-        K.upsample_concat(y, skip, cat)
         t1 = ws.get("dec_t1", (n_img, H, W, hid), torch.bfloat16, dev)
-        _cbr(cat, dec, ca, ba, t1)
+        _upconv_bn_relu(y, skip, dec, ca, ba, ws, t1)
         t2 = ws.get("dec_t2_%d" % H, (n_img, H, W, hid), torch.bfloat16, dev)
         _cbr(t1, dec, cb, bb, t2)
         y = t2
         if feats is not None:
             feats.append(t2)
-        _count(1)
     if getattr(dec, "interpolate_before_seg", False):          # reference lib/mask_predictor.py:88-97
         fine = c1
         for on, (cname, bname, mul_) in ((True, ("conv2_1", "bn1_1", 2)), (getattr(dec, "seg_last", False), ("conv1_0", "bn1_0", 4))):
             if not on:
                 continue
             H, W = mul_ * fine.shape[1], mul_ * fine.shape[2]
-            up = ws.get("dec_up_%d" % mul_, (n_img, H, W, hid), torch.bfloat16, dev)
-            K.upsample_nhwc(y, up)
-            y = ws.get("dec_y_%d" % mul_, (n_img, H, W, hid), torch.bfloat16, dev)
-            _cbr(up, dec, cname, bname, y)
-            _count(1)
+            out = ws.get("dec_y_%d" % mul_, (n_img, H, W, hid), torch.bfloat16, dev)
+            _upconv_bn_relu(y, None, dec, cname, bname, ws, out)
+            y = out
     _, H, W, _ = y.shape
     w11 = dec.prepared.get("w11", [dec.conv1_1.weight], lambda: _f32(dec.conv1_1.weight.reshape(2, -1)))
     lg = ws.get("dec_logits", (n_img, H, W, 2), torch.float32, dev)
