@@ -21,7 +21,7 @@
 extern "C" {
 #endif
 
-#define LAVT_ABI_VERSION 3
+#define LAVT_ABI_VERSION 4
 
 #define LAVT_ERR_SHAPE 1
 #define LAVT_ERR_CUDA 2
@@ -314,14 +314,27 @@ int lavt_layernorm_window_gather_bwd(const float* x, int32_t C, const lavt_win_g
 int lavt_patch_merge_layernorm_bwd(const float* x, int32_t B, int32_t D, int32_t H, int32_t W, int32_t C, const void* dy_bf16,
                                    const float* gamma, float eps, float* dx, float* dgamma, float* dbeta, void* stream);
 /* Adjoint of lavt_window_attention: qkv / out as saved by the forward, dout = gradient of out; dqkv bf16 [rows, 3C] = gradient
- * of the UNSCALED qkv projection; dtable_t fp32 [nH, L] accumulates the relative_position_bias_table gradient (transposed).
- * lse: the row statistics saved by lavt_window_attention_lse, or NULL (then they are recomputed in a first pass).
- * Windows of up to ~400 tokens (shared-memory resident). */
+ * of the UNSCALED qkv projection; dtable_t fp32 [nH, L] accumulates the relative_position_bias_table gradient (transposed), or NULL.
+ * lse: the row statistics saved by lavt_window_attention_lse, or NULL (then they are recomputed in a first pass; mma.sync kernel only).
+ * Windows of any size up to 8 x 12 x 12 = 1152 tokens; lavt_window_attention_bwd_kernel tells which kernel a geometry gets.
+ * workspace: fp32 scratch of at least lavt_window_attention_bwd_workspace_floats(geom, L, nH) floats, owned by the caller and
+ * not read across calls (NULL / 0 where that query returns 0).  Nothing is allocated inside the call. */
 int lavt_window_attention_bwd(const void* qkv, const void* out, const void* dout, const float* table_t, int32_t L, int32_t nH,
-                              const lavt_win_geom_t* geom, const float* lse, void* dqkv, float* dtable_t, void* stream);
-/* Kernel selection for lavt_window_attention_bwd (process-wide; initial value from LAVT_ATTN_BWD_IMPL = mma | tc):
- *   0 = auto: the tcgen05 / TMEM kernel (attn_bwd_tc.cu) for 7 x 7 windows with an even number of frames when lse is given, else mma.sync
- *   1 = mma.sync kernel only (attn_bwd.cu)      2 = same as auto.   Returns the previous setting. */
+                              const lavt_win_geom_t* geom, const float* lse, void* dqkv, float* dtable_t, float* workspace,
+                              int64_t workspace_floats, void* stream);
+/* fp32 workspace lavt_window_attention_bwd needs for this geometry when lse is given: 0 except on attn_bwd_tc2.cu for windows of more
+ * than 128 tokens (one [N rounded up to 128, 32] dQ scratch per CTA of the persistent grid) */
+int64_t lavt_window_attention_bwd_workspace_floats(const lavt_win_geom_t* geom, int32_t L, int32_t nH);
+/* The kernel lavt_window_attention_bwd runs for this geometry under the current selection (host arithmetic, no device call):
+ * 1 = mma.sync (attn_bwd.cu), 2 = attn_bwd_tc.cu, 3 = attn_bwd_tc2.cu, 0 = none (the call fails with LAVT_ERR_SHAPE). */
+int lavt_window_attention_bwd_kernel(const lavt_win_geom_t* geom, int32_t L, int32_t nH, int32_t has_lse);
+/* Kernel selection for lavt_window_attention_bwd (process-wide; initial value from LAVT_ATTN_BWD_IMPL = mma | tc | tc2):
+ *   0 = auto: attn_bwd_tc.cu (tcgen05 / TMEM) for 7 x 7 windows with an even number of frames when lse is given, else the mma.sync
+ *       kernel (attn_bwd.cu) where Q / K / V / dO and the table fit its shared memory, else attn_bwd_tc2.cu (tcgen05 / TMEM, key tiles
+ *       outer, any window of 16 ... 1152 tokens with lse: the full and large clamped 8 x 12 x 12 windows)
+ *   1 = mma.sync kernel only      2 = same as auto
+ *   3 = attn_bwd_tc2.cu wherever it applies (A/B runs and tests), else as auto
+ * Any other value means auto.  Returns the previous setting. */
 int lavt_set_attention_bwd_impl(int32_t impl);
 
 /* ---- PWAM + LanguageGate backward (adjoints of lavt_pwam_* above; reference lib/video_swin_transformer.py:919-1009, 519-525) ---- */

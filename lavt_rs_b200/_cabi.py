@@ -68,7 +68,7 @@ def lib() -> C.CDLL:
     return l
 
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 _i32, _i64, _f32, _vp = C.c_int32, C.c_int64, C.c_float, C.c_void_p
 _EP = C.POINTER(Epilogue)
@@ -120,7 +120,7 @@ SIGNATURES = {
     "lavt_layernorm_rows_bwd": [_vp, _i64, _i64, _i32, _vp, _i64, _vp, _f32, _vp, _vp, _vp, _vp, _vp],
     "lavt_layernorm_window_gather_bwd": [_vp, _i32, _WG, _vp, _vp, _f32, _vp, _vp, _vp, _vp, _vp],
     "lavt_patch_merge_layernorm_bwd": [_vp, _i32, _i32, _i32, _i32, _i32, _vp, _vp, _f32, _vp, _vp, _vp, _vp],
-    "lavt_window_attention_bwd": [_vp, _vp, _vp, _vp, _i32, _i32, _WG, _vp, _vp, _vp, _vp],
+    "lavt_window_attention_bwd": [_vp, _vp, _vp, _vp, _i32, _i32, _WG, _vp, _vp, _vp, _vp, _i64, _vp],
     "lavt_pwam_attend_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _i32, _i32, _i32, _vp],
     "lavt_pwam_mul_norm_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _vp],
     "lavt_instnorm_bwd": [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i32, _i64, _i32, _vp],
@@ -158,6 +158,7 @@ SIGNATURES = {
 }
 EXPORTS = ["lavt_last_error", "lavt_abi_version", "lavt_instnorm_workspace_floats", "lavt_set_attention_impl", "lavt_set_attention_bwd_impl",
            "lavt_gemm_splitk_workspace_floats", "lavt_conv3x3_wgrad_workspace_floats", "lavt_gacd_workspace_floats", "lavt_conv3d_wgrad_workspace_floats", "lavt_adamw_chunk_elems", "lavt_window_attention_has_lse",
+           "lavt_window_attention_bwd_kernel", "lavt_window_attention_bwd_workspace_floats",
            *SIGNATURES.keys()]
 
 
@@ -169,6 +170,10 @@ def _declare(l: C.CDLL) -> None:
     l.lavt_gemm_splitk_workspace_floats.restype = C.c_int64
     l.lavt_window_attention_has_lse.argtypes = [_WG, _i32, _i32]
     l.lavt_window_attention_has_lse.restype = C.c_int
+    l.lavt_window_attention_bwd_kernel.argtypes = [_WG, _i32, _i32, _i32]
+    l.lavt_window_attention_bwd_kernel.restype = C.c_int
+    l.lavt_window_attention_bwd_workspace_floats.argtypes = [_WG, _i32, _i32]
+    l.lavt_window_attention_bwd_workspace_floats.restype = C.c_int64
     l.lavt_conv3x3_wgrad_workspace_floats.argtypes = [_i32, _i32, _i32, _i32, _i32]
     l.lavt_conv3x3_wgrad_workspace_floats.restype = C.c_int64
     l.lavt_conv3d_wgrad_workspace_floats.argtypes = [_i32, _i32, _i32, _i32, _i32, _i32]
@@ -438,11 +443,30 @@ def set_attention_impl(impl: str) -> str:
     return {v: k for k, v in codes.items()}.get(prev, "auto")
 
 
+ATTN_BWD_IMPLS = ("auto", "mma", "tc", "tc2")
+ATTN_BWD_KERNELS = {0: None, 1: "mma", 2: "tc", 3: "tc2"}
+
+
 def set_attention_bwd_impl(impl: str) -> str:
-    """'auto' / 'tc' (tcgen05 kernel attn_bwd_tc.cu where it applies) or 'mma' (mma.sync kernel only); returns the previous setting."""
-    names = ["auto", "mma", "tc"]
-    prev = lib().lavt_set_attention_bwd_impl(names.index(impl))
-    return names[prev] if 0 <= prev < len(names) else "auto"
+    """'auto' / 'tc' (tcgen05 kernel attn_bwd_tc.cu for 7 x 7 windows, else the mma.sync kernel where the window fits its shared
+    memory, else the tcgen05 kernel attn_bwd_tc2.cu), 'mma' (mma.sync kernel only) or 'tc2' (attn_bwd_tc2.cu wherever it applies, else
+    as auto); returns the previous setting."""
+    if impl not in ATTN_BWD_IMPLS:
+        raise LavtError(f"attention backward impl must be one of {list(ATTN_BWD_IMPLS)}, not {impl!r}")
+    prev = lib().lavt_set_attention_bwd_impl(ATTN_BWD_IMPLS.index(impl))
+    return ATTN_BWD_IMPLS[prev] if 0 <= prev < len(ATTN_BWD_IMPLS) else "auto"
+
+
+def window_attention_bwd_kernel(table_t: torch.Tensor, geom: WinGeom, has_lse: bool = True) -> Optional[str]:
+    """The kernel window_attention_bwd runs for this geometry under the current selection: 'mma', 'tc', 'tc2', or None (no kernel)."""
+    nH, L = table_t.shape
+    return ATTN_BWD_KERNELS[int(lib().lavt_window_attention_bwd_kernel(C.byref(geom), L, nH, 1 if has_lse else 0))]
+
+
+def window_attention_bwd_workspace_floats(table_t: torch.Tensor, geom: WinGeom) -> int:
+    """fp32 elements of the workspace window_attention_bwd needs for this geometry (with lse); 0 for most windows."""
+    nH, L = table_t.shape
+    return int(lib().lavt_window_attention_bwd_workspace_floats(C.byref(geom), L, nH))
 
 
 def window_attention_has_lse(table_t: torch.Tensor, geom: WinGeom) -> bool:
@@ -791,14 +815,22 @@ def patch_merge_layernorm_bwd(x, B, D, H, W, dy, gamma, dx, dgamma, dbeta, eps: 
                                                stream_ptr()), "lavt_patch_merge_layernorm_bwd")
 
 
-def window_attention_bwd(qkv, out, dout, table_t, geom: WinGeom, dqkv, dtable_t, lse=None) -> None:
-    """Adjoint of window_attention; dtable_t fp32 [nH, L] accumulates; lse = the forward's row statistics or None (recomputed)."""
+def window_attention_bwd(qkv, out, dout, table_t, geom: WinGeom, dqkv, dtable_t, lse=None, workspace=None) -> None:
+    """Adjoint of window_attention; dtable_t fp32 [nH, L] accumulates (or None); lse = the forward's row statistics or None
+    (recomputed).  workspace: fp32 scratch of at least window_attention_bwd_workspace_floats(table_t, geom) elements, or None: then
+    one is allocated here when this geometry needs it (pass a reused buffer for CUDA-graph capture)."""
     nH, L = table_t.shape
+    if workspace is None:
+        need = window_attention_bwd_workspace_floats(table_t, geom) if lse is not None else 0
+        if need > 0:
+            workspace = torch.empty(need, dtype=torch.float32, device=qkv.device)
     t0 = TIMER.begin()
     check(lib().lavt_window_attention_bwd(_c(qkv, torch.bfloat16, "qkv").data_ptr(), _c(out, torch.bfloat16, "out").data_ptr(),
                                           _c(dout, torch.bfloat16, "dout").data_ptr(), _c(table_t, torch.float32, "table_t").data_ptr(),
                                           L, nH, C.byref(geom), ptr(lse), _c(dqkv, torch.bfloat16, "dqkv").data_ptr(),
-                                          ptr(dtable_t), stream_ptr()), "lavt_window_attention_bwd")
+                                          ptr(dtable_t), None if workspace is None else _c(workspace, torch.float32, "workspace").data_ptr(),
+                                          0 if workspace is None else workspace.numel(), stream_ptr()),
+          "lavt_window_attention_bwd")
     rows = geom.rows()
     TIMER.end(t0, "window_attn_bwd_kernel", 12.0 * rows * geom.N * nH * 32, 2.0 * rows * nH * 32 * 8, f"rows{rows} N{geom.N} nH{nH}")
 

@@ -377,23 +377,47 @@ __global__ void __launch_bounds__(AB_WARPS * 32, 1) window_attn_bwd_kernel(const
 int attn_bwd_impl_setting(int set) {
   static int impl = -1;
   if (impl < 0) {
-    const char* e = getenv("LAVT_ATTN_BWD_IMPL");      // "mma" = mma.sync kernel only, "tc" = tcgen05 kernel where it applies (= auto)
-    impl = !e ? 0 : e[0] == 'm' ? 1 : e[0] == 't' ? 2 : 0;
+    // "mma" = mma.sync kernel only, "tc" = attn_bwd_tc.cu where it applies (= auto), "tc2" = attn_bwd_tc2.cu wherever it applies
+    const char* e = getenv("LAVT_ATTN_BWD_IMPL");
+    impl = !e ? 0 : e[0] == 'm' ? 1 : (e[0] == 't' && e[1] == 'c' && e[2] == '2') ? 3 : e[0] == 't' ? 2 : 0;
   }
   const int prev = impl;
-  if (set >= 0) impl = set <= 2 ? set : 0;
+  if (set >= 0) impl = set <= 3 ? set : 0;
   return prev;
 }
 
-int window_attn_bwd_dispatch(const AttnBwdParams& p, cudaStream_t st) {
+static size_t ab_smem_bytes(const AttnBwdParams& p) {
+  const int NP = (p.win.N + 15) / 16 * 16;
+  return static_cast<size_t>(NP) * 64 * 4 + static_cast<size_t>(NP) * sizeof(AbTok) + static_cast<size_t>(p.L) * 12 + 32;
+}
+
+AttnBwdKernel window_attn_bwd_choose(const AttnBwdParams& p) {
+  const WinGeom& w = p.win;
+  if (p.C != p.nH * AB_HD || w.N <= 0 || w.N != w.wd * w.wh * w.ww) return AttnBwdKernel::NONE;
+  const int impl = attn_bwd_impl_setting(-1);
+  if (impl == 3 && window_attn_bwd_tc2_supported(p)) return AttnBwdKernel::TC2;
+  if (impl != 1 && window_attn_bwd_tc_supported(p)) return AttnBwdKernel::TC;
+  if (ab_smem_bytes(p) <= 227 * 1024) return AttnBwdKernel::MMA;
+  if (impl != 1 && window_attn_bwd_tc2_supported(p)) return AttnBwdKernel::TC2;
+  return AttnBwdKernel::NONE;
+}
+
+long long window_attn_bwd_workspace_floats(const AttnBwdParams& p) {
+  return window_attn_bwd_choose(p) == AttnBwdKernel::TC2 ? window_attn_bwd_tc2_workspace_floats(p) : 0;
+}
+
+int window_attn_bwd_dispatch(const AttnBwdParams& p, float* workspace, long long workspace_floats, cudaStream_t st) {
   const WinGeom& w = p.win;
   LAVT_REQUIRE(p.C == p.nH * AB_HD, "attention backward: head_dim must be 32 (C=%d, heads=%d)", p.C, p.nH);
   LAVT_REQUIRE(w.N > 0 && w.N == w.wd * w.wh * w.ww, "attention backward: bad window geometry");
-  if (attn_bwd_impl_setting(-1) != 1 && window_attn_bwd_tc_supported(p)) return window_attn_bwd_tc_dispatch(p, st);
+  const AttnBwdKernel k = window_attn_bwd_choose(p);
+  if (k == AttnBwdKernel::TC) return window_attn_bwd_tc_dispatch(p, st);
+  if (k == AttnBwdKernel::TC2) return window_attn_bwd_tc2_dispatch(p, workspace, workspace_floats, st);
+  const size_t smem = ab_smem_bytes(p);
+  LAVT_REQUIRE(k == AttnBwdKernel::MMA, "attention backward: no kernel for a window of %d tokens (table %d, %s): the mma.sync kernel "
+               "needs %zu B of shared memory, the tcgen05 kernels need 16 ... 1152 tokens and the forward's saved lse%s", w.N, p.L,
+               p.lse ? "lse saved" : "no lse", smem, attn_bwd_impl_setting(-1) == 1 ? " (mma.sync only was selected)" : "");
   const int NP = (w.N + 15) / 16 * 16;
-  const size_t smem = static_cast<size_t>(NP) * 64 * 4 + static_cast<size_t>(NP) * sizeof(AbTok) + static_cast<size_t>(p.L) * 12 + 32;
-  LAVT_REQUIRE(smem <= 227 * 1024, "attention backward: window of %d tokens (table %d) needs %zu B of shared memory; windows above ~400 "
-               "tokens (8x12x12) are not supported by the training path yet", w.N, p.L, smem);
   static size_t configured = 0;
   if (smem > configured) {
     LAVT_CUDA(cudaFuncSetAttribute(window_attn_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));

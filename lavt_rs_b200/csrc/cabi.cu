@@ -190,7 +190,7 @@ int lavt_window_attention_has_lse(const lavt_win_geom_t* geom, int32_t L, int32_
   return window_attn_choose(p) != AttnKernel::MMA ? 1 : 0;
 }
 
-int lavt_set_attention_bwd_impl(int32_t impl) { return attn_bwd_impl_setting(impl >= 0 && impl <= 2 ? impl : 0); }
+int lavt_set_attention_bwd_impl(int32_t impl) { return attn_bwd_impl_setting(impl >= 0 && impl <= 3 ? impl : 0); }
 int lavt_set_attention_impl(int32_t impl) { return attn_impl_setting(impl == 3 || impl == 4 ? impl : 0); }
 
 int64_t lavt_instnorm_workspace_floats(int32_t B, int64_t n, int32_t C) { return colstats_workspace_floats(B, n, C); }
@@ -513,17 +513,39 @@ int lavt_patch_merge_layernorm_bwd(const float* x, int32_t B, int32_t D, int32_t
   return ln_bwd_dispatch(MODE_MERGE, p, S(stream));
 }
 
-int lavt_window_attention_bwd(const void* qkv, const void* out, const void* dout, const float* table_t, int32_t L, int32_t nH,
-                              const lavt_win_geom_t* geom, const float* lse, void* dqkv, float* dtable_t, void* stream) {
-  LAVT_REQUIRE(geom != nullptr, "attention backward: geometry is NULL");
+static AttnBwdParams attn_bwd_params(const lavt_win_geom_t* geom, int32_t L, int32_t nH) {
   AttnBwdParams p;
   std::memset(&p, 0, sizeof(p));
   std::memcpy(&p.win, geom, sizeof(WinGeom));
-  p.qkv = CB(qkv); p.out = CB(out); p.dout = CB(dout); p.table_t = table_t; p.dqkv = MB(dqkv); p.dtable_t = dtable_t; p.lse = lse;
   p.C = nH * 32; p.nH = nH; p.L = L;
   p.qscale = 0.17677669529663687f;      // 32^-0.5
+  return p;
+}
+
+int lavt_window_attention_bwd(const void* qkv, const void* out, const void* dout, const float* table_t, int32_t L, int32_t nH,
+                              const lavt_win_geom_t* geom, const float* lse, void* dqkv, float* dtable_t, float* workspace,
+                              int64_t workspace_floats, void* stream) {
+  LAVT_REQUIRE(geom != nullptr, "attention backward: geometry is NULL");
+  AttnBwdParams p = attn_bwd_params(geom, L, nH);
+  p.qkv = CB(qkv); p.out = CB(out); p.dout = CB(dout); p.table_t = table_t; p.dqkv = MB(dqkv); p.dtable_t = dtable_t; p.lse = lse;
   LAVT_REQUIRE(L == (2 * p.win.Wd - 1) * (2 * p.win.Wh - 1) * (2 * p.win.Ww - 1), "attention backward: table length %d does not match the window", L);
-  return window_attn_bwd_dispatch(p, S(stream));
+  return window_attn_bwd_dispatch(p, workspace, workspace_floats, S(stream));
+}
+
+int lavt_window_attention_bwd_kernel(const lavt_win_geom_t* geom, int32_t L, int32_t nH, int32_t has_lse) {
+  if (geom == nullptr) return 0;
+  static const float lse_tag = 0.f;      // only compared against NULL: the choice is host arithmetic
+  AttnBwdParams p = attn_bwd_params(geom, L, nH);
+  if (has_lse) p.lse = &lse_tag;
+  return static_cast<int>(window_attn_bwd_choose(p));
+}
+
+int64_t lavt_window_attention_bwd_workspace_floats(const lavt_win_geom_t* geom, int32_t L, int32_t nH) {
+  if (geom == nullptr) return 0;
+  static const float lse_tag = 0.f;
+  AttnBwdParams p = attn_bwd_params(geom, L, nH);
+  p.lse = &lse_tag;                      // the training path always saves lse; without it no kernel with a workspace applies
+  return window_attn_bwd_workspace_floats(p);
 }
 
 int lavt_pwam_attend_bwd(const float* qpre, const float* stats, const float* k, const float* v, const float* mask, const void* do_bf16,

@@ -64,11 +64,24 @@ struct AttnBwdParams {
   float qscale;                // hd^-0.5
   WinGeom win;
 };
-int window_attn_bwd_dispatch(const AttnBwdParams& p, cudaStream_t st);
+// workspace: fp32 scratch of window_attn_bwd_workspace_floats(p) floats (only attn_bwd_tc2.cu uses one)
+int window_attn_bwd_dispatch(const AttnBwdParams& p, float* workspace, long long workspace_floats, cudaStream_t st);
+// set < 0: query only; returns the previous value (0 = auto, 1 = mma.sync only, 2 = attn_bwd_tc.cu where it applies (= auto),
+// 3 = attn_bwd_tc2.cu wherever it applies)
+int attn_bwd_impl_setting(int set);
+// The kernel window_attn_bwd_dispatch runs for p (host arithmetic only, no device call): attn_bwd_tc.cu (full 7 x 7 windows with an even
+// frame count), the mma.sync kernel of attn_bwd.cu (windows whose Q / K / V / dO and table fit its shared memory: <= 496 tokens at w12),
+// attn_bwd_tc2.cu (every other window of 16 ... 1152 tokens with saved lse), or NONE (no kernel: the dispatcher raises)
+enum class AttnBwdKernel { NONE = 0, MMA = 1, TC = 2, TC2 = 3 };
+AttnBwdKernel window_attn_bwd_choose(const AttnBwdParams& p);
+long long window_attn_bwd_workspace_floats(const AttnBwdParams& p);
 // tcgen05 / TMEM variant (attn_bwd_tc.cu): 7 x 7 windows with an even number of frames and the forward's saved row statistics
-int attn_bwd_impl_setting(int set);   // set < 0: query only; returns the previous value (0 = auto, 1 = mma.sync only, 2 = tcgen05 where it applies)
 bool window_attn_bwd_tc_supported(const AttnBwdParams& p);
 int window_attn_bwd_tc_dispatch(const AttnBwdParams& p, cudaStream_t st);
+// tcgen05 / TMEM variant for any window of 16 ... 1152 tokens (attn_bwd_tc2.cu): key tiles outer, dQ partials through an fp32 scratch
+bool window_attn_bwd_tc2_supported(const AttnBwdParams& p);
+long long window_attn_bwd_tc2_workspace_floats(const AttnBwdParams& p);
+int window_attn_bwd_tc2_dispatch(const AttnBwdParams& p, float* workspace, long long workspace_floats, cudaStream_t st);
 
 struct LnBwdParams {
   const float* x;              // LN input rows (fp32, pitch ldx), gathered like the forward

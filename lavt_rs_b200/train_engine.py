@@ -307,7 +307,9 @@ def swin_block_bwd(blk, saved, dx: torch.Tensor, grads: GradStore, ws: Workspace
     linear_bwd(dyw, att, blk.attn.proj.weight, blk.attn.proj.bias, grads, ws, pw, "proj", dx_bf16=datt, bias_done=fusep)
     dqkv = ws.get("bw_dqkv", (rows, 3 * C), torch.bfloat16, dev)
     tbl = blk.attn.relative_position_bias_table
-    K.window_attention_bwd(qkv, att, datt, table_t, geom, dqkv, grads.table_t(tbl) if tbl.requires_grad else None, lse=lse)
+    nws = K.window_attention_bwd_workspace_floats(table_t, geom) if lse is not None else 0
+    aws = ws.get("bw_attn", (nws,), torch.float32, dev) if nws > 0 else None
+    K.window_attention_bwd(qkv, att, datt, table_t, geom, dqkv, grads.table_t(tbl) if tbl.requires_grad else None, lse=lse, workspace=aws)
     dxw = ws.get("bw_dxw", (rows, C), torch.bfloat16, dev)
     linear_bwd(dqkv, xw, blk.attn.qkv.weight, blk.attn.qkv.bias, grads, ws, pw, "qkv", dx_bf16=dxw)
     K.layernorm_window_gather_bwd(x0, geom, dxw, blk.norm1.weight, dx, grads.of(blk.norm1.weight), grads.of(blk.norm1.bias),

@@ -13,7 +13,8 @@ Mirrors the inner loop of the reference's ``train_one_epoch_*`` (train.py:330-36
   (replaces DistributedDataParallel, train.py:590-593).
 
 Stochastic depth (DropPath) runs as a per-sample scale inside the proj / fc2 GEMM epilogues.  Not implemented in training mode
-(raise, no fallback): --hs / --version variants, windows above ~400 tokens (8x12x12).  The 2-D image models
+(raise, no fallback): --hs / --version variants.  Every window size trains, the 8 x 12 x 12 windows of --window12 included
+(attention backward of windows over ~500 tokens on the tcgen05 kernel attn_bwd_tc2.cu, with a workspace from ``engine.Workspace``).  The 2-D image models
 (lavt / lavt_one) train through the same code with one frame per clip.  The text encoder's own backward runs through the stock ``transformers``
 module under autograd (SURVEY.md section 8f-2 marks the text side as the next row, not the hot path).
 """

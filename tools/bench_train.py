@@ -3,6 +3,7 @@
 4 clips (8x384x384) per GPU, gradient all-reduce over NCCL at N > 1.
 
     python tools/bench_train.py --steps 5 --warmup 2
+    python tools/bench_train.py --window12 --graph           # the (8,12,12)-window model (attention backward on attn_bwd_tc2.cu)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/bench_train.py --gpus 2
 
 One step = what the reference's ``train_one_epoch_ytvos`` does per iteration up to the optimizer (train.py:430-470):
@@ -35,6 +36,7 @@ def main():
     p.add_argument("--frozen-text", action="store_true", help="do not backpropagate into the text encoder")
     p.add_argument("--optimizer", action="store_true", help="include the AdamW update (FusedAdamW over the reference's parameter groups, "
                                                             "poly LR) in the timed step")
+    p.add_argument("--window12", action="store_true", help="(8,12,12) windows instead of the default (8,7,7)")
     p.add_argument("--sep-t-pwam", action="store_true", help="the reference README's video configuration (SepTPWAM fusion flags)")
     p.add_argument("--no-overlap-allreduce", dest="overlap_allreduce", action="store_false",
                    help="all-reduce after the backward instead of launching each stage's all-reduce under the rest of the backward (default)")
@@ -66,7 +68,7 @@ def main():
     K.check(K.lib().lavt_check_device(), "lavt_check_device")
 
     B0.SEP_T_PWAM = bool(a.sep_t_pwam)
-    model = B0.build_model(False, dev).train()
+    model = B0.build_model(a.window12, dev).train()
     for layer in model.backbone.layers:
         for blk in layer.blocks:
             blk.drop_path_rate = 0.0
@@ -264,7 +266,7 @@ def main():
 
     total = Bc * world
     value = total * a.steps / (ms * 1e-3)
-    flops_clip = 3.0 * (2074.8e9 - 3.4e9 + (1043.6e9 if a.sep_t_pwam else 0.0))          # forward + input gradients + weight gradients of every contraction
+    flops_clip = 3.0 * (B0.flops_per_clip(a.window12) - 3.4e9)          # forward + input gradients + weight gradients of every contraction
     g = fam.get("gemm_bf16_tc_kernel", {"launches": 0, "ms": 0.0, "flops": 0.0})
     ab = fam.get("window_attn_bwd_kernel", {"launches": 0, "ms": 0.0, "flops": 0.0})
     af = fam.get("window_attn_kernel", {"launches": 0, "ms": 0.0, "flops": 0.0})
@@ -275,7 +277,7 @@ def main():
         "warmup": max(a.warmup, 3), "ms_per_step": ms / a.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "bf16", "data": "synthetic",
         "config": {"workload": "LAVT-RS Video Swin-B training step: BERT-base + backbone + decoder forward, [0.9,1.1]-weighted CE, backward, "
-                               "gradient all-reduce; 8x384x384 clips, 20-token expression, window 8x7x7, DropPath off, no optimizer update",
+                               "gradient all-reduce; 8x384x384 clips, 20-token expression, window " + ("8x12x12" if a.window12 else "8x7x7") + ", DropPath off, no optimizer update",
                    "clips_per_gpu_per_step": Bc, "global_clips_per_step": total,
                    "parallelism": f"data-parallel x{world}" + ((", NCCL gradient all-reduce (" + ("per stage, under the backward" if a.overlap_allreduce else "after the backward") + ") + SyncBN statistics") if world > 1 else ""),
                    "text_encoder": "frozen" if a.frozen_text else ("transformers BertModel under autograd (fp32)" + ("" if a.eager_text else ", forward and backward replayed as CUDA graphs")),
@@ -286,7 +288,7 @@ def main():
                      "bound": "tensor", "achieved": achieved, "peak": peak, "unit": "TFLOP/s", "frac": achieved / peak if peak else None,
                      "peak_kind": pk_kind + " sustained cuBLAS bf16", "traffic": None, "launches": g["launches"], "ms_per_step": g["ms"],
                      "alg_flops_per_step": g["flops"],
-                     "attention_bwd": {"kernel": "window_attn_bwd_tc_kernel (tcgen05 / TMEM; 7 x 7 windows with saved row statistics) / window_attn_bwd_kernel (mma.sync, other windows)", "launches": ab["launches"], "ms_per_step": ab["ms"],
+                     "attention_bwd": {"kernel": "window_attn_bwd_tc_kernel (tcgen05 / TMEM; 7 x 7 windows with saved row statistics) / window_attn_bwd_kernel (mma.sync, windows that fit its shared memory) / window_attn_bwd_tc2_kernel (tcgen05 / TMEM; larger windows, e.g. 8 x 12 x 12)", "launches": ab["launches"], "ms_per_step": ab["ms"],
                                        "tflops": ab["flops"] / (ab["ms"] * 1e-3) / 1e12 if ab["ms"] > 0 else 0.0},
                      "attention_fwd": {"launches": af["launches"], "ms_per_step": af["ms"]},
                      "whole_step_tflops": flops_clip * value / world / 1e12},
@@ -294,7 +296,7 @@ def main():
     if a.cpu_baseline and world == 1:
         from oracle import lavt_oracle as O
         torch.set_num_threads(os.cpu_count() or 1)
-        cfg = O.OracleConfig.swin("base", window12=False, video=True)
+        cfg = O.OracleConfig.swin("base", window12=a.window12, video=True)
         sd = {k: v.detach().float().cpu().requires_grad_(v.is_floating_point() and "running" not in k) for k, v in model.state_dict().items()}
         x, ids, m = B0.synth_batch(1, 100)
         tgt = torch.randint(0, 2, (B0.T_FRAMES, B0.IMG, B0.IMG))
